@@ -11,6 +11,7 @@ csrc/dist.cu), with grouped NCCL send/recv only as the fallback transport (MARLI
 
   python bench.py [--gpus N] [--steps K] [--warmup W] [--size S]          (N>1: launched by torchrun)
   python bench.py --impl reference ...   CPU restatement of the reference path (oracle port) on host cores
+  python bench.py --dump-outputs DIR ... also write the last timed step's product to DIR/C.npy (see dump_outputs)
 
 Prints ONE JSON line on rank 0.
 """
@@ -40,6 +41,7 @@ os.environ.setdefault("CUDA_DEVICE_MAX_CONNECTIONS", "32")     # one hardware qu
 FP64_PEAK_TFLOPS_MEASURED = 37.1   # scripts/dmma_bench.cu on this pool's B200 (profiles/r01_probe_*): 148 SM x 64 DFMA/clk x 1.965 GHz
 METRIC = "fp64 dense multiply throughput (2*N^3 flop), 16384x16384 BlockMatrix 2x2 grid"
 METRIC_TALL = "fp64 tall-skinny multiply throughput (2*M*K*N flop), DenseVecMatrix 1048576x1024 x 1024x1024"
+DUMP_MAX_DIM = 2048                # --dump-outputs: at most 2048 x 2048 fp64 = 32 MiB
 
 
 def parse():
@@ -62,7 +64,15 @@ def parse():
     ap.add_argument("--ref-seconds", type=float, default=3.0, help="target seconds per step of --impl reference")
     ap.add_argument("--no-parity", action="store_true")
     ap.add_argument("--no-extra-configs", action="store_true")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write the product of the last one as DIR/C.npy (fp64, or fp32 for bf16 tiles); "
+                         f"a product with more than {DUMP_MAX_DIM} rows or columns is written on a fixed seeded sample of them")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the GPU path's product; --impl reference times a host-dependent sample of the workload")
+    return args
 
 
 # ------------------------------------------------------------------------------------------ CPU arm
@@ -86,12 +96,11 @@ def cpu_port_sample(size: int, grid: int, target_seconds: float, steps: int = 5,
     """The reference algorithm on host cores (oracle port, numpy/OpenBLAS dgemm on all threads), on a BOUNDED
     sample of the workload: one of the (grid^3) block products A(0,0) * B(0,0)[:, :w], w chosen so a step takes
     about `target_seconds` — or, for the tall-skinny workload, a slice of the rows of one partition times the broadcast
-    1024 x 1024 matrix (DenseVecMatrix.scala:1660-1680).  Median of >= 5 timed steps after a warm-up.
+    1024 x 1024 matrix (DenseVecMatrix.scala:1660-1680).  Median of `steps` timed steps after a warm-up.
     Returns a dict: value (TFLOP/s), threads (actually used), cores (host), sample, ms, extrapolation."""
     import numpy as np
     from oracle import reference_model as rm
     threads, blas = cpu_threads()
-    steps = max(5, steps)
     bs = size // grid
     rng = np.random.default_rng(42)
     probe = 2048
@@ -204,7 +213,7 @@ def run_reference(args):
     if rank != 0:
         return
     tall = args.workload == "tallskinny"
-    r = cpu_port_sample(args.size, args.grid, args.ref_seconds, steps=max(5, args.steps), warmup=max(1, min(2, args.warmup)), tall=tall)
+    r = cpu_port_sample(args.size, args.grid, args.ref_seconds, steps=args.steps, warmup=max(1, min(2, args.warmup)), tall=tall)
     tf = r["value"]
     line = {
         "impl": "reference", "metric": metric_name(args), "value": tf, "unit": "TFLOP/s", "n_gpus": args.gpus, "steps": args.steps,
@@ -336,6 +345,53 @@ def freivalds_rows(A_rows, B, C_rows, ws, tol, probes=3):
     worst = float(t.item())
     return {"max_scaled_err": worst, "tol": tol, "ok": bool(worst <= tol), "probes": probes, "n_ranks": ws,
             "method": "Freivalds on device per row shard: C v vs A (B v) with torch/cuBLAS dgemv; max_i |y-z|_i / (|A||B||v|)_i, worst rank"}
+
+
+def dump_indices(M: int, N: int):
+    """The rows and columns of an M x N product that --dump-outputs writes: all of them up to DUMP_MAX_DIM, else a fixed
+    seeded sample of DUMP_MAX_DIM, sorted."""
+    import numpy as np
+    rng = np.random.default_rng(20261017)
+    return tuple(np.sort(rng.choice(n, DUMP_MAX_DIM, replace=False)) if n > DUMP_MAX_DIM else np.arange(n) for n in (M, N))
+
+
+def dump_outputs(out_dir: Path, Cm, M: int, N: int, tall: bool, bf16: bool, ws: int, rank: int):
+    """Write the product C (M x N) a caller of the timed path receives as out_dir/C.npy, restricted to dump_indices(M, N),
+    so that two builds run with the same arguments (hence the same seeded inputs) can be compared element for element.
+    Every rank copies the sampled elements of the C tiles / row shard it holds into a zero matrix and the pieces are
+    summed onto rank 0 (each element of C is held by exactly one rank)."""
+    import numpy as np
+    import torch
+    import torch.distributed as dist
+    rows, cols = dump_indices(M, N)
+    dev = torch.device("cuda", torch.cuda.current_device())
+    out = torch.zeros(len(rows), len(cols), dtype=torch.float32 if bf16 else torch.float64, device=dev)
+    cidx = torch.from_numpy(cols).to(dev)
+    if tall:
+        ids = np.asarray(Cm.ids)
+        if len(ids):
+            order = np.argsort(ids, kind="stable")
+            pos = np.minimum(np.searchsorted(ids[order], rows), len(ids) - 1)
+            hit = ids[order][pos] == rows
+            s = Cm.data
+            shard = s.buf[: s.rows * s.cols].view(s.rows, s.cols)                 # row-major shard
+            src = torch.from_numpy(order[pos[hit]]).to(dev)
+            out[torch.from_numpy(np.nonzero(hit)[0]).to(dev)] = shard.index_select(0, src).index_select(1, cidx).to(out.dtype)
+    else:
+        bm, bn = -(-M // Cm.numBlksByRow()), -(-N // Cm.numBlksByCol())
+        for b, s in Cm.blocks:
+            ri = np.nonzero((rows >= b.row * bm) & (rows < b.row * bm + s.rows))[0]
+            ci = np.nonzero((cols >= b.column * bn) & (cols < b.column * bn + s.cols))[0]
+            if len(ri) and len(ci):
+                tile = s.buf[: s.rows * s.cols].view(s.cols, s.rows).t()          # packed column-major tile
+                piece = tile.index_select(0, torch.from_numpy(rows[ri] - b.row * bm).to(dev))
+                piece = piece.index_select(1, torch.from_numpy(cols[ci] - b.column * bn).to(dev))
+                out[ri[0]: ri[-1] + 1, ci[0]: ci[-1] + 1] = piece.to(out.dtype)
+    if ws > 1:
+        dist.all_reduce(out)
+    if rank == 0:
+        out_dir.mkdir(parents=True, exist_ok=True)
+        np.save(out_dir / "C.npy", out.cpu().numpy())
 
 
 # ------------------------------------------------------------------------------------------ the other BASELINE configs
@@ -754,6 +810,8 @@ def run_ours(args):
             parity = freivalds_rows(A.data, B, Cm.data, ws, tol)
         else:
             parity = freivalds_blockmatrix(A, B, Cm, ws, tol)
+    if args.dump_outputs:
+        dump_outputs(Path(args.dump_outputs), Cm, rows_total if tall else N, kdim if tall else N, tall, bf16, ws, rank)
     del Cm
 
     # ---- the other BASELINE configurations, in the same run (only next to the default headline workload) ----

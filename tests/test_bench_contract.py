@@ -32,7 +32,7 @@ def test_reference_arm_line():
     cb = d["cpu_baseline"]
     assert cb["kind"] == "port" and cb["cores"] >= 1 and cb["value"] == d["value"] and cb["sample"]
     assert d["e2e"] == {"value": d["value"], "unit": d["unit"], "h2d_bytes_per_step": 0, "d2h_bytes_per_step": 0}
-    assert cb["extrapolation"]["by"] == "flops" and "median of" in cb["sample"]
+    assert cb["extrapolation"]["by"] == "flops" and "median of 1 after" in cb["sample"]      # --steps sets the timed steps
 
 
 def test_reference_arm_thread_count_survives_torchrun_env():
@@ -77,3 +77,11 @@ def test_reference_arm_tallskinny_workload():
     d = _run(["--impl", "reference", "--workload", "tallskinny", "--steps", "1", "--warmup", "1", "--ref-seconds", "0.3"])
     assert "tall-skinny" in d["metric"] and "configs[3]" in d["config"]["workload"]
     assert d["value"] > 0 and "rows" in d["cpu_baseline"]["sample"] and d["cpu_baseline"]["f2j_single_thread"]["cores"] == 1
+
+
+def test_bad_arguments_are_refused():
+    """No timed steps, or a dump of the CPU arm (its sample depends on the host's speed), is a usage error."""
+    for args in (["--impl", "reference", "--steps", "0"], ["--impl", "reference", "--dump-outputs", "out"]):
+        out = subprocess.run([sys.executable, str(ROOT / "bench.py"), *args], stdout=subprocess.PIPE, stderr=subprocess.PIPE,
+                             text=True, timeout=300, cwd=ROOT)
+        assert out.returncode == 2 and "error:" in out.stderr and not out.stdout, args

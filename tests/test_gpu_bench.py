@@ -5,6 +5,7 @@ import subprocess
 import sys
 from pathlib import Path
 
+import numpy as np
 import pytest
 
 pytestmark = pytest.mark.gpu
@@ -31,3 +32,23 @@ def test_gpu_arm_line_small_config():
     assert 0 < e["value"] < d["value"]                               # host buffers in and out cannot beat the resident number
     assert d["gpu_launches"] >= 3
     assert "sm_mhz" in d["clocks"] and "reasons" in d["clocks"]
+
+
+def test_dump_outputs_is_the_last_product(oracle, tmp_path):
+    """--dump-outputs writes C = A*B of the timed path on the rows and columns bench.dump_indices samples (2100 > 2048:
+    the sampled case), the inputs being the seeded generator streams the oracle restates."""
+    import bench
+    n = 2100
+    out = subprocess.run([sys.executable, str(ROOT / "bench.py"), "--size", str(n), "--grid", "2", "--steps", "2", "--warmup", "1",
+                          "--no-cpu-baseline", "--no-int8-split", "--no-e2e", "--dump-outputs", str(tmp_path)],
+                         stdout=subprocess.PIPE, stderr=subprocess.PIPE, text=True, timeout=600)
+    assert out.returncode == 0, out.stderr[-3000:]
+    assert json.loads([l for l in out.stdout.splitlines() if l.startswith("{")][0])["steps"] == 2
+    assert sorted(p.name for p in tmp_path.iterdir()) == ["C.npy"]
+    got = np.load(tmp_path / "C.npy")
+    r, c = bench.dump_indices(n, n)
+    A = oracle.random_block_matrix(n, n, 2, 2, seed=42).to_breeze()
+    B = oracle.random_block_matrix(n, n, 2, 2, seed=43).to_breeze()
+    want = A[r] @ B[:, c]                                            # U[0,1) inputs: |A||B| = A B
+    assert got.dtype == np.float64 and got.shape == (bench.DUMP_MAX_DIM, bench.DUMP_MAX_DIM)
+    assert (np.abs(got - want) / want).max() <= 1e-10

@@ -255,20 +255,12 @@ def _parse_plain(text):
     return np.array([rows[i] for i in sorted(rows)])
 
 
-def test_reference_tool_output_loads(oracle, golden_dir, tmp_path):
-    """Files written by the reference's own tools/generateMatrix.cpp (compiled into oracle/_ref/, see oracle/Makefile):
-    the committed run, and a live run when the binary is present, load through the oracle's and the product's
-    loadMatrixFile (utils/MTUtils.scala:286-300) to exactly the values printed."""
-    import subprocess
-    from pathlib import Path
+def test_reference_tool_output_loads(oracle, golden_dir):
+    """Files written by the reference's own tools/generateMatrix.cpp (two stored runs, see tests/golden/make_generated.sh)
+    load through the oracle's and the product's loadMatrixFile (utils/MTUtils.scala:286-300) to exactly the values
+    printed."""
     import marlin_b200 as mb
-    paths = [golden_dir / "generated.9.6"]
-    tool = Path(__file__).resolve().parents[1] / "oracle" / "_ref" / "generateMatrix"
-    if tool.exists():
-        live = tmp_path / "live.11.3"
-        live.write_text(subprocess.run([str(tool), "11", "3"], check=True, stdout=subprocess.PIPE, text=True).stdout)
-        paths.append(live)
-    for p in paths:
+    for p in (golden_dir / "generated.9.6", golden_dir / "generated.11.3"):
         want = _parse_plain(p.read_text())
         assert want.shape in ((9, 6), (11, 3)) and (want >= 0).all() and (want <= 5).all()
         assert np.array_equal(oracle.load_matrix_file(str(p)).to_breeze(), want)
