@@ -298,6 +298,53 @@ int32_t mb_matmul_blocked_dist_host(mb_comm* comm, const double* const* A_host, 
 int32_t mb_host_alloc_shared(const char* name, int64_t bytes, void** out);
 int32_t mb_host_free_shared(const char* name, void* ptr, int64_t bytes, int32_t unlink_name);
 
+/* ---- sparse blocks: `new SubMatrix(spMatrix = ...)` (matrix/SubMatrix.scala:22-25) holding a SparseMatrix
+ *      (matrix/Matrices.scala:136-253).  An mb_spblock is CSC on the device, the reference's one SparseVector per column:
+ *      col_ptr int32[cols+1] (col_ptr[0] = 0, non-decreasing; an empty column has col_ptr[c] == col_ptr[c+1]),
+ *      row_idx int32[nnz] strictly increasing within each column and inside [0, rows), val fp64[nnz].
+ *      The products write a dense column-major result (a dense mb_block, any view), as the reference does.  Each output
+ *      element is a sequential sum from +0.0 in the reference's order with one rounded multiply and one rounded add per
+ *      term (the JVM never fuses them); accumulate = 1 adds the finished sum to C with one rounding, i.e. exactly
+ *      mb_block_add of a separate product (the k-way reduceByKey of matrix/BlockMatrix.scala:177). ---- */
+typedef struct mb_spblock mb_spblock;
+/* The validation mb_spblock_upload runs before anything is uploaded (pure host logic): MB_ERR_INVALID_ARG for a
+ * col_ptr that does not start at 0 or decreases, or a row index out of range or not strictly increasing in its column. */
+int32_t mb_csc_check(int32_t rows, int32_t cols, const int32_t* col_ptr, const int32_t* row_idx);
+int32_t mb_spblock_upload(mb_ctx* ctx, int32_t rows, int32_t cols, const int32_t* col_ptr, const int32_t* row_idx,
+                          const double* val, mb_spblock** out);
+/* host arrays of cols+1, nnz and nnz entries */
+int32_t mb_spblock_download(mb_ctx* ctx, const mb_spblock* sp, int32_t* col_ptr, int32_t* row_idx, double* val);
+int32_t mb_spblock_info(const mb_spblock* sp, int32_t* rows, int32_t* cols, int64_t* nnz);
+int32_t mb_spblock_free(mb_ctx* ctx, mb_spblock* sp);
+/* A new block with the same structure and values (the scalar ops of SubMatrix.scala:52-58,71-85,121-129 map a copy). */
+int32_t mb_spblock_copy(mb_ctx* ctx, const mb_spblock* sp, mb_spblock** out);
+/* The stored values as a non-owning (nnz x 1) fp64 mb_block, so mb_block_axpb / mb_block_div map them in place:
+ * the scalar ops touch the stored values only (A + 1 leaves implicit zeros at zero). */
+int32_t mb_spblock_values(mb_ctx* ctx, mb_spblock* sp, mb_block** out);
+/* SparseMatrix.toDense (matrix/Matrices.scala:106-119): out (rows x cols fp64, any view) := the dense matrix. */
+int32_t mb_spblock_to_dense(mb_ctx* ctx, const mb_spblock* sp, mb_block* out);
+/* SparseMatrix.rand(rows, cols, sparsity) (matrix/Matrices.scala:157-173): every column holds exactly
+ * count = (int)(cols * sparsity) distinct rows (the count follows numCols, as in the reference), sorted, values U[0,1).
+ * The reference draws from an unseeded java.util.Random; here column c of a block seeded with `partition_seed` (one of
+ * mb_partition_seeds, as dense blocks are seeded) has its own splitmix64 stream, rows are chosen by selection sampling,
+ * so a seed reproduces the matrix.  Generated on the device.  mb_sparse_rand_count is the count and its checks:
+ * MB_ERR_INVALID_ARG for a negative or NaN sparsity, a count above rows (where the reference loops forever) or
+ * count * cols >= 2^31 (matrix/Matrices.scala:71). */
+int32_t mb_sparse_rand_count(int32_t rows, int32_t cols, double sparsity, int32_t* count);
+int32_t mb_spblock_rand(mb_ctx* ctx, int32_t rows, int32_t cols, double sparsity, int64_t partition_seed, mb_spblock** out);
+/* SubMatrix.multiply, (dense, sparse) arm (SubMatrix.scala:95-97) -> LibMatrixMult.multDenseSparse
+ * (matrix/LibMatrixMult.scala:15-41): C(r,j) = sum over B's column j in stored order of B(k,j)*A(r,k); a column holding
+ * exactly one entry equal to 1.0 copies A's column (:28-29).  MB_ERR_DIM_MISMATCH "matrix dimension mismatch: a v.s b". */
+int32_t mb_spmm_dense_sparse(mb_ctx* ctx, const mb_block* A, const mb_spblock* B, mb_block* C, int32_t accumulate);
+/* SubMatrix.multiply, (sparse, dense) arms (SubMatrix.scala:98-100,112-114) -> LibMatrixMult.multSparseDense
+ * (matrix/LibMatrixMult.scala:43-77) AS DEFINED: C(r,j) = sum over k ascending of A(r,k)*B(k,j) over the stored A(r,k).
+ * The reference's loop indexes B with `i * cd + bi` (:60) and is only right for K <= 32 and N <= 32 (DESIGN.md,
+ * documented deviations); B's offset / ld / transpose are honoured as mb_block_gemm honours them. */
+int32_t mb_spmm_sparse_dense(mb_ctx* ctx, const mb_spblock* A, const mb_block* B, mb_block* C, int32_t accumulate);
+/* SubMatrix.multiply, (sparse, sparse) arm (SubMatrix.scala:92-94) -> SparseMatrix.multiply (matrix/Matrices.scala:122-152):
+ * C(r,j) = sum over B's column j in stored order of B(k,j)*A(r,k), over the stored A(r,k). */
+int32_t mb_spgemm_to_dense(mb_ctx* ctx, const mb_spblock* A, const mb_spblock* B, mb_block* C, int32_t accumulate);
+
 /* ---- rows <-> blocks on device (matrix/DenseVecMatrix.scala:1084-1223, 1259-1328;
  *      matrix/BlockMatrix.scala:575-594): a DenseVecMatrix shard is a row-major (rows x cols)
  *      buffer, i.e. a transposed block; these are strided copies (mb_block_copy on views). */

@@ -101,11 +101,75 @@ struct BlockID {
     int hashCode() const { return row * 31 + column + seq; }
 };
 
+// ---------------------------------------------------------------------------------------------- SparseMatrix
+// matrix/Matrices.scala:136-253 — a CSC block on the device (mb_spblock).  The products return dense blocks.
+struct SparseVector {                                                                   // Vectors.sparse(size, indices, values)
+    int size = 0;
+    std::vector<int32_t> indices;
+    std::vector<double> values;
+};
+class SubMatrix;
+class SparseMatrix {
+public:
+    SparseMatrix() = default;
+    SparseMatrix(int numRows, int numCols, const std::vector<SparseVector>& values) {     // one vector per column
+        if ((int)values.size() != numCols) throw std::invalid_argument("SparseMatrix: one SparseVector per column");
+        std::vector<int32_t> cp(1, 0), ri;
+        std::vector<double> v;
+        for (const auto& sv : values) {
+            if (sv.indices.size() != sv.values.size()) throw std::invalid_argument("SparseVector: indices / values differ in length");
+            ri.insert(ri.end(), sv.indices.begin(), sv.indices.end());
+            v.insert(v.end(), sv.values.begin(), sv.values.end());
+            cp.push_back((int32_t)ri.size());
+        }
+        *this = fromCSC(numRows, numCols, cp, ri, v);
+    }
+    static SparseMatrix fromCSC(int numRows, int numCols, const std::vector<int32_t>& colPtr, const std::vector<int32_t>& rowIdx,
+                                const std::vector<double>& val) {
+        if ((int)colPtr.size() != numCols + 1) throw std::invalid_argument("SparseMatrix: col_ptr needs numCols + 1 entries");
+        mb_spblock* h = nullptr;
+        check(mb_spblock_upload(Context::get(), numRows, numCols, colPtr.data(), rowIdx.data(), val.data(), &h));
+        return SparseMatrix(h);
+    }
+    // Matrices.scala:236-253 on the device, seeded (see mb_spblock_rand)
+    static SparseMatrix rand(int numRows, int numCols, double sparsity, int64_t seed) {
+        mb_spblock* h = nullptr;
+        check(mb_spblock_rand(Context::get(), numRows, numCols, sparsity, seed, &h));
+        return SparseMatrix(h);
+    }
+    int numRows() const { int32_t r = 0; mb_spblock_info(h_.get(), &r, nullptr, nullptr); return r; }
+    int numCols() const { int32_t c = 0; mb_spblock_info(h_.get(), nullptr, &c, nullptr); return c; }
+    int64_t nnz() const { int64_t n = 0; mb_spblock_info(h_.get(), nullptr, nullptr, &n); return n; }
+    mb_spblock* handle() const { return h_.get(); }
+    explicit operator bool() const { return (bool)h_; }
+    inline SubMatrix toDense() const;                                                     // :185-198
+    inline SubMatrix multiply(const SparseMatrix& o) const;                               // :208-231
+    // the scalar ops of SubMatrix.scala:52-58,71-85,121-129: a copy whose stored values are alpha*v + beta (or v / b)
+    SparseMatrix mapValues(double alpha, double beta, bool divide = false, double b = 1.0) const {
+        mb_spblock* h = nullptr;
+        check(mb_spblock_copy(Context::get(), h_.get(), &h));
+        SparseMatrix out(h);
+        if (nnz() > 0) {
+            mb_block *src = nullptr, *dst = nullptr;
+            check(mb_spblock_values(Context::get(), h_.get(), &src));
+            std::shared_ptr<mb_block> s(src, [](mb_block* p) { mb_block_free(Context::get(), p); });
+            check(mb_spblock_values(Context::get(), h, &dst));
+            std::shared_ptr<mb_block> d(dst, [](mb_block* p) { mb_block_free(Context::get(), p); });
+            check(divide ? mb_block_div(Context::get(), src, b, 0, dst) : mb_block_axpb(Context::get(), src, alpha, beta, dst));
+        }
+        return out;
+    }
+private:
+    explicit SparseMatrix(mb_spblock* h) : h_(h, [](mb_spblock* p) { mb_spblock_free(Context::get(), p); }) {}
+    std::shared_ptr<mb_spblock> h_;
+};
+
 // ---------------------------------------------------------------------------------------------- SubMatrix
-// matrix/SubMatrix.scala — the per-block value type, device resident (dense branch; sparse is out of scope).
+// matrix/SubMatrix.scala — the per-block value type, device resident: a dense block, or a sparse one (spMatrix).
 class SubMatrix {
 public:
     SubMatrix() = default;
+    explicit SubMatrix(const SparseMatrix& spMatrix) : sp_(spMatrix) {}                 // new SubMatrix(spMatrix = ...)
     explicit SubMatrix(const DenseMatrix& m) {                                        // new SubMatrix(denseMatrix = ...)
         mb_block* b = nullptr;
         check(mb_block_upload(Context::get(), m.data.data(), 0, m.rows, m.cols, std::max(1, m.rows), 0, MB_F64, &b));
@@ -126,10 +190,20 @@ public:
         s.own(b);
         return s;
     }
-    int rows() const { int r = 0; mb_block_info(h_.get(), &r, nullptr, nullptr, nullptr, nullptr, nullptr); return r; }
-    int cols() const { int c = 0; mb_block_info(h_.get(), nullptr, &c, nullptr, nullptr, nullptr, nullptr); return c; }
-    bool isSparse() const { return false; }
-    mb_block* handle() const { return h_.get(); }
+    int rows() const {
+        if (sp_) return sp_.numRows();
+        int r = 0; mb_block_info(h_.get(), &r, nullptr, nullptr, nullptr, nullptr, nullptr); return r;
+    }
+    int cols() const {
+        if (sp_) return sp_.numCols();
+        int c = 0; mb_block_info(h_.get(), nullptr, &c, nullptr, nullptr, nullptr, nullptr); return c;
+    }
+    bool isSparse() const { return (bool)sp_; }
+    const SparseMatrix& sparseBlock() const { return sp_; }
+    mb_block* handle() const {
+        if (sp_) throw std::invalid_argument("this operation needs a dense block and this block is sparse: convert with toDenseBlocks");
+        return h_.get();
+    }
 
     SubMatrix t() const {                                                             // Breeze `.t`: a view
         mb_block* v = nullptr;
@@ -141,21 +215,33 @@ public:
         check(mb_block_slice(Context::get(), h_.get(), r0, r1, c0, c1, &v));
         return view(v);
     }
-    SubMatrix add(const SubMatrix& o) const { SubMatrix r = empty(rows(), cols()); check(mb_block_add(Context::get(), h_.get(), o.h_.get(), r.h_.get())); return r; }        // :41-45
-    SubMatrix add(double b) const { SubMatrix r = empty(rows(), cols()); check(mb_block_axpb(Context::get(), h_.get(), 1.0, b, r.h_.get())); return r; }                    // :52-58
-    SubMatrix subtract(const SubMatrix& o) const { SubMatrix r = empty(rows(), cols()); check(mb_block_sub(Context::get(), h_.get(), o.h_.get(), r.h_.get())); return r; }   // :60-64
-    SubMatrix subtract(double b) const { SubMatrix r = empty(rows(), cols()); check(mb_block_axpb(Context::get(), h_.get(), 1.0, -b, r.h_.get())); return r; }              // :71-77
-    SubMatrix divide(double b) const { SubMatrix r = empty(rows(), cols()); check(mb_block_div(Context::get(), h_.get(), b, 0, r.h_.get())); return r; }                     // :79-85
-    SubMatrix multiply(double b) const { SubMatrix r = empty(rows(), cols()); check(mb_block_axpb(Context::get(), h_.get(), b, 0.0, r.h_.get())); return r; }               // :123-131
+    SubMatrix add(const SubMatrix& o) const { densePair(o, "add"); SubMatrix r = empty(rows(), cols()); check(mb_block_add(Context::get(), h_.get(), o.h_.get(), r.h_.get())); return r; }        // :41-45
+    SubMatrix add(double b) const { if (sp_) return SubMatrix(sp_.mapValues(1.0, b)); SubMatrix r = empty(rows(), cols()); check(mb_block_axpb(Context::get(), h_.get(), 1.0, b, r.h_.get())); return r; }                    // :52-58
+    SubMatrix subtract(const SubMatrix& o) const { densePair(o, "subtract"); SubMatrix r = empty(rows(), cols()); check(mb_block_sub(Context::get(), h_.get(), o.h_.get(), r.h_.get())); return r; }   // :60-64
+    SubMatrix subtract(double b) const { if (sp_) return SubMatrix(sp_.mapValues(1.0, -b)); SubMatrix r = empty(rows(), cols()); check(mb_block_axpb(Context::get(), h_.get(), 1.0, -b, r.h_.get())); return r; }              // :71-77
+    SubMatrix divide(double b) const { if (sp_) return SubMatrix(sp_.mapValues(1.0, 0.0, true, b)); SubMatrix r = empty(rows(), cols()); check(mb_block_div(Context::get(), h_.get(), b, 0, r.h_.get())); return r; }                     // :79-85
+    SubMatrix multiply(double b) const { if (sp_) return SubMatrix(sp_.mapValues(b, 0.0)); SubMatrix r = empty(rows(), cols()); check(mb_block_axpb(Context::get(), h_.get(), b, 0.0, r.h_.get())); return r; }               // :123-131
     SubMatrix elementMultiply(const SubMatrix& o) const { SubMatrix r = empty(rows(), cols()); check(mb_block_hadamard(Context::get(), h_.get(), o.h_.get(), r.h_.get())); return r; }
-    SubMatrix multiply(const SubMatrix& o) const {                                    // :87-91 -> dgemm
+    SubMatrix multiply(const SubMatrix& o) const {                                    // :87-91 -> dgemm; sparse arms :92-100
+        if (sp_ || o.sp_) {
+            SubMatrix r = empty(rows(), o.cols());
+            multiplyInto(o, r, false);
+            return r;
+        }
         if (cols() != o.rows())
             throw std::invalid_argument("Dimension mismatch during matrix-matrix multiplication: " + std::to_string(cols()) + " vs " + std::to_string(o.rows()));
         SubMatrix r = empty(rows(), o.cols());
         check(mb_block_gemm(Context::get(), h_.get(), o.h_.get(), r.h_.get(), 0));
         return r;
     }
-    void multiplyInto(const SubMatrix& o, SubMatrix& out, bool accumulate) const { check(mb_block_gemm(Context::get(), h_.get(), o.h_.get(), out.h_.get(), accumulate ? 1 : 0)); }
+    void multiplyInto(const SubMatrix& o, SubMatrix& out, bool accumulate) const {
+        const int acc = accumulate ? 1 : 0;
+        if (sp_ && o.sp_) check(mb_spgemm_to_dense(Context::get(), sp_.handle(), o.sp_.handle(), out.handle(), acc));          // :92-94
+        else if (o.sp_) check(mb_spmm_dense_sparse(Context::get(), handle(), o.sp_.handle(), out.handle(), acc));               // :95-97
+        else if (sp_) check(mb_spmm_sparse_dense(Context::get(), sp_.handle(), o.handle(), out.handle(), acc));                 // :98-100
+        else check(mb_block_gemm(Context::get(), h_.get(), o.h_.get(), out.h_.get(), acc));
+    }
+    SubMatrix toDenseBlock() const { return sp_ ? sp_.toDense() : *this; }           // BlockMatrix.scala:598
     SubMatrix transpose() const {                                                     // denseBlock.t.copy (BlockMatrix.scala:517)
         SubMatrix r = empty(cols(), rows());
         check(mb_block_transpose(Context::get(), h_.get(), r.h_.get()));
@@ -192,6 +278,7 @@ public:
     void assign(const SubMatrix& src) { check(mb_block_copy(Context::get(), src.h_.get(), h_.get())); }   // this(range) := src
     double sum() const { double s = 0; check(mb_block_sum(Context::get(), h_.get(), &s)); return s; }
     DenseMatrix denseBlock() const {                                                  // collect to the host (toBreeze)
+        if (sp_) return sp_.toDense().denseBlock();
         DenseMatrix m(rows(), cols());
         check(mb_block_download(Context::get(), h_.get(), m.data.data(), std::max(1, m.rows)));
         return m;
@@ -204,7 +291,30 @@ private:
         s.h_ = std::shared_ptr<mb_block>(v, [parent](mb_block* p) { mb_block_free(Context::get(), p); });
         return s;
     }
+    void densePair(const SubMatrix& o, const char* op) const {                      // :46-48, :66-68
+        if (sp_ || o.sp_)
+            throw std::invalid_argument(std::string("Not supported ") + op + "-operator between matrices of sparsity with " +
+                                        (sp_ ? "true" : "false") + " and " + (o.sp_ ? "true" : "false"));
+    }
     std::shared_ptr<mb_block> h_;
+    SparseMatrix sp_;
+};
+
+inline SubMatrix SparseMatrix::toDense() const {
+    SubMatrix r = SubMatrix::empty(numRows(), numCols());
+    check(mb_spblock_to_dense(Context::get(), h_.get(), r.handle()));
+    return r;
+}
+inline SubMatrix SparseMatrix::multiply(const SparseMatrix& o) const { return SubMatrix(*this).multiply(SubMatrix(o)); }
+
+// matrix/LibMatrixMult.scala
+struct LibMatrixMult {
+    static SubMatrix multDenseSparse(const SubMatrix& denseMat, const SparseMatrix& sparseMat) {        // :15-41
+        return denseMat.multiply(SubMatrix(sparseMat));
+    }
+    static SubMatrix multSparseDense(const SparseMatrix& sparseMat, const SubMatrix& denseMat) {        // :43-77, as defined
+        return SubMatrix(sparseMat).multiply(denseMat);
+    }
 };
 
 class DenseVecMatrix;

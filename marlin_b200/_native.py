@@ -25,6 +25,7 @@ _LIB_PATH = Path(__file__).resolve().parent / "lib" / "libmarlin_b200.so"
 
 c_ctx = C.c_void_p
 c_blk = C.c_void_p
+c_sp = C.c_void_p          # mb_spblock*
 c_i32 = C.c_int32
 c_i64 = C.c_int64
 c_f64 = C.c_double
@@ -114,6 +115,19 @@ SIGNATURES = {
     "mb_host_free_shared": (c_i32, [C.c_char_p, C.c_void_p, c_i64, c_i32]),
     "mb_matmul_blocked_dist": (c_i32, [C.c_void_p, C.POINTER(c_blk), C.POINTER(c_i32), C.POINTER(c_blk), C.POINTER(c_i32), c_i32, c_i32,
                                        c_i32, C.POINTER(c_i32), C.POINTER(c_i32), C.POINTER(c_i32), c_i32, C.POINTER(c_blk)]),
+    "mb_csc_check": (c_i32, [c_i32, c_i32, C.POINTER(c_i32), C.POINTER(c_i32)]),
+    "mb_spblock_upload": (c_i32, [c_ctx, c_i32, c_i32, C.POINTER(c_i32), C.POINTER(c_i32), c_dp, C.POINTER(c_sp)]),
+    "mb_spblock_download": (c_i32, [c_ctx, c_sp, C.POINTER(c_i32), C.POINTER(c_i32), c_dp]),
+    "mb_spblock_info": (c_i32, [c_sp, C.POINTER(c_i32), C.POINTER(c_i32), C.POINTER(c_i64)]),
+    "mb_spblock_free": (c_i32, [c_ctx, c_sp]),
+    "mb_spblock_copy": (c_i32, [c_ctx, c_sp, C.POINTER(c_sp)]),
+    "mb_spblock_values": (c_i32, [c_ctx, c_sp, C.POINTER(c_blk)]),
+    "mb_spblock_to_dense": (c_i32, [c_ctx, c_sp, c_blk]),
+    "mb_sparse_rand_count": (c_i32, [c_i32, c_i32, c_f64, C.POINTER(c_i32)]),
+    "mb_spblock_rand": (c_i32, [c_ctx, c_i32, c_i32, c_f64, c_i64, C.POINTER(c_sp)]),
+    "mb_spmm_dense_sparse": (c_i32, [c_ctx, c_blk, c_sp, c_blk, c_i32]),
+    "mb_spmm_sparse_dense": (c_i32, [c_ctx, c_sp, c_blk, c_blk, c_i32]),
+    "mb_spgemm_to_dense": (c_i32, [c_ctx, c_sp, c_sp, c_blk, c_i32]),
 }
 
 

@@ -16,7 +16,7 @@ CSRC = PKG / "csrc"
 LIBDIR = PKG / "lib"
 LIB = LIBDIR / "libmarlin_b200.so"
 
-SOURCES = ["capi.cu", "gemm_f64.cu", "gemm_bf16.cu", "gemm_ozaki.cu", "elementwise.cu", "blas12.cu", "peer.cu", "dist.cu", "factor.cu", "hostlogic.cpp"]
+SOURCES = ["capi.cu", "gemm_f64.cu", "gemm_bf16.cu", "gemm_ozaki.cu", "elementwise.cu", "blas12.cu", "peer.cu", "dist.cu", "factor.cu", "sparse.cu", "hostlogic.cpp"]
 NVCC_FLAGS = [
     "-gencode", "arch=compute_100a,code=sm_100a",
     "-lineinfo", "-O3", "-std=c++17",

@@ -8,6 +8,7 @@
 #include "gemm_ozaki.h"
 #include "blas12.h"
 #include "factor.h"
+#include "sparse.h"
 
 #include <cuda_runtime.h>
 #include <algorithm>
@@ -1211,4 +1212,188 @@ int32_t mb_fill_uniform(mb_ctx* ctx, mb_block* blk, int64_t partition_seed, int6
     return MB_OK;
 }
 
+// ---------------------------------------------------------------------------------- sparse blocks
+// `new SubMatrix(spMatrix = ...)` (matrix/SubMatrix.scala:22-25): CSC device arrays; see include/marlin_b200.h.
+static int32_t spblock_alloc(mb_ctx* ctx, int32_t rows, int32_t cols, long long nnz, mb_spblock** out) {
+    mb_spblock* sp = new (std::nothrow) mb_spblock();
+    if (!sp) return fail(MB_ERR_OOM, "host allocation failed");
+    sp->rows = rows; sp->cols = cols; sp->nnz = nnz; sp->device = ctx->device;
+    cudaError_t e = cudaMalloc(&sp->col_ptr, sizeof(int) * ((size_t)cols + 1));
+    if (e == cudaSuccess && nnz > 0) e = cudaMalloc(&sp->row_idx, sizeof(int) * (size_t)nnz);
+    if (e == cudaSuccess && nnz > 0) e = cudaMalloc(&sp->val, sizeof(double) * (size_t)nnz);
+    if (e != cudaSuccess) { mb_spblock_free(ctx, sp); *out = nullptr; return cuda_fail(e, "cudaMalloc(sparse block)"); }
+    *out = sp;
+    return MB_OK;
+}
+
+static int32_t dense_f64(const mb_block* b, const char* what) {
+    if (b->dtype != MB_F64) return fail(MB_ERR_UNSUPPORTED, "%s: fp64 dense blocks only", what);
+    return MB_OK;
+}
+
+static int32_t check_out(const mb_block* C, int rows, int cols, const char* what) {
+    if (!C) return fail(MB_ERR_INVALID_ARG, "%s: null result block", what);
+    if (C->dtype != MB_F64) return fail(MB_ERR_UNSUPPORTED, "%s: the result block must be fp64", what);
+    if (C->rows != rows || C->cols != cols)
+        return fail(MB_ERR_DIM_MISMATCH, "%s: result block is %dx%d, expected %dx%d", what, C->rows, C->cols, rows, cols);
+    return MB_OK;
+}
+
+// per-call workspace of the tile pointers of the scatter products: stream-ordered, released on the same stream
+struct tile_ws {
+    int* p = nullptr;
+    cudaStream_t st;
+    ~tile_ws() { if (p) cudaFreeAsync(p, st); }
+};
+
+int32_t mb_spblock_upload(mb_ctx* ctx, int32_t rows, int32_t cols, const int32_t* col_ptr, const int32_t* row_idx,
+                          const double* val, mb_spblock** out) {
+    MB_CTX(ctx);
+    if (!out) return fail(MB_ERR_INVALID_ARG, "mb_spblock_upload: null output");
+    int32_t r = mb_csc_check(rows, cols, col_ptr, row_idx);
+    if (r) return r;
+    const long long nnz = col_ptr[cols];
+    if (nnz > 0 && !val) return fail(MB_ERR_INVALID_ARG, "mb_spblock_upload: null values");
+    r = spblock_alloc(ctx, rows, cols, nnz, out);
+    if (r) return r;
+    mb_spblock* sp = *out;
+    cudaError_t e = cudaMemcpyAsync(sp->col_ptr, col_ptr, sizeof(int) * ((size_t)cols + 1), cudaMemcpyHostToDevice, ctx->stream);
+    if (e == cudaSuccess && nnz > 0)
+        e = cudaMemcpyAsync(sp->row_idx, row_idx, sizeof(int) * (size_t)nnz, cudaMemcpyHostToDevice, ctx->stream);
+    if (e == cudaSuccess && nnz > 0)
+        e = cudaMemcpyAsync(sp->val, val, sizeof(double) * (size_t)nnz, cudaMemcpyHostToDevice, ctx->stream);
+    if (e == cudaSuccess) e = cudaStreamSynchronize(ctx->stream);
+    if (e != cudaSuccess) { mb_spblock_free(ctx, sp); *out = nullptr; return cuda_fail(e, "mb_spblock_upload"); }
+    return MB_OK;
+}
+
+int32_t mb_spblock_download(mb_ctx* ctx, const mb_spblock* sp, int32_t* col_ptr, int32_t* row_idx, double* val) {
+    MB_CTX(ctx);
+    if (!sp || !col_ptr || (sp->nnz > 0 && (!row_idx || !val))) return fail(MB_ERR_INVALID_ARG, "mb_spblock_download: null argument");
+    MB_CUDA(cudaMemcpyAsync(col_ptr, sp->col_ptr, sizeof(int) * ((size_t)sp->cols + 1), cudaMemcpyDeviceToHost, ctx->stream));
+    if (sp->nnz > 0) {
+        MB_CUDA(cudaMemcpyAsync(row_idx, sp->row_idx, sizeof(int) * (size_t)sp->nnz, cudaMemcpyDeviceToHost, ctx->stream));
+        MB_CUDA(cudaMemcpyAsync(val, sp->val, sizeof(double) * (size_t)sp->nnz, cudaMemcpyDeviceToHost, ctx->stream));
+    }
+    MB_CUDA(cudaStreamSynchronize(ctx->stream));
+    return MB_OK;
+}
+
+int32_t mb_spblock_info(const mb_spblock* sp, int32_t* rows, int32_t* cols, int64_t* nnz) {
+    if (!sp) return fail(MB_ERR_INVALID_ARG, "null sparse block");
+    if (rows) *rows = sp->rows;
+    if (cols) *cols = sp->cols;
+    if (nnz) *nnz = sp->nnz;
+    return MB_OK;
+}
+
+int32_t mb_spblock_free(mb_ctx* ctx, mb_spblock* sp) {
+    if (!sp) return MB_OK;
+    if (ctx) cudaSetDevice(ctx->device);
+    cudaFree(sp->col_ptr);
+    cudaFree(sp->row_idx);
+    cudaFree(sp->val);
+    delete sp;
+    return MB_OK;
+}
+
+int32_t mb_spblock_copy(mb_ctx* ctx, const mb_spblock* sp, mb_spblock** out) {
+    MB_CTX(ctx);
+    if (!sp || !out) return fail(MB_ERR_INVALID_ARG, "mb_spblock_copy: null argument");
+    int32_t r = spblock_alloc(ctx, sp->rows, sp->cols, sp->nnz, out);
+    if (r) return r;
+    mb_spblock* d = *out;
+    cudaError_t e = cudaMemcpyAsync(d->col_ptr, sp->col_ptr, sizeof(int) * ((size_t)sp->cols + 1), cudaMemcpyDeviceToDevice,
+                                    ctx->stream);
+    if (e == cudaSuccess && sp->nnz > 0)
+        e = cudaMemcpyAsync(d->row_idx, sp->row_idx, sizeof(int) * (size_t)sp->nnz, cudaMemcpyDeviceToDevice, ctx->stream);
+    if (e == cudaSuccess && sp->nnz > 0)
+        e = cudaMemcpyAsync(d->val, sp->val, sizeof(double) * (size_t)sp->nnz, cudaMemcpyDeviceToDevice, ctx->stream);
+    if (e != cudaSuccess) { mb_spblock_free(ctx, d); *out = nullptr; return cuda_fail(e, "mb_spblock_copy"); }
+    return MB_OK;
+}
+
+int32_t mb_spblock_values(mb_ctx* ctx, mb_spblock* sp, mb_block** out) {
+    if (!sp) return fail(MB_ERR_INVALID_ARG, "null sparse block");
+    return mb_block_wrap(ctx, sp->val, 0, int32_t(sp->nnz), 1, int32_t(sp->nnz > 0 ? sp->nnz : 1), 0, MB_F64, out);
+}
+
+int32_t mb_spblock_to_dense(mb_ctx* ctx, const mb_spblock* sp, mb_block* out) {
+    MB_CTX(ctx);
+    if (!sp) return fail(MB_ERR_INVALID_ARG, "mb_spblock_to_dense: null sparse block");
+    int32_t r = check_out(out, sp->rows, sp->cols, "toDense");
+    if (r) return r;
+    int launches = 0;
+    MB_CUDA(mb::sparse_to_dense(sp->col_ptr, sp->row_idx, sp->val, sp->rows, sp->cols, f64_ptr(out), rs(out), cs(out),
+                                ctx->stream, &launches));
+    ctx->launches += launches;
+    return MB_OK;
+}
+
+int32_t mb_spblock_rand(mb_ctx* ctx, int32_t rows, int32_t cols, double sparsity, int64_t partition_seed, mb_spblock** out) {
+    MB_CTX(ctx);
+    if (!out) return fail(MB_ERR_INVALID_ARG, "mb_spblock_rand: null output");
+    int32_t count = 0;
+    int32_t r = mb_sparse_rand_count(rows, cols, sparsity, &count);
+    if (r) return r;
+    r = spblock_alloc(ctx, rows, cols, (long long)count * cols, out);
+    if (r) return r;
+    int launches = 0;
+    cudaError_t e = mb::sparse_rand(rows, cols, count, (unsigned long long)partition_seed, (*out)->col_ptr, (*out)->row_idx,
+                                    (*out)->val, ctx->stream, &launches);
+    ctx->launches += launches;
+    if (e != cudaSuccess) { mb_spblock_free(ctx, *out); *out = nullptr; return cuda_fail(e, "mb_spblock_rand"); }
+    return MB_OK;
+}
+
+int32_t mb_spmm_dense_sparse(mb_ctx* ctx, const mb_block* A, const mb_spblock* B, mb_block* C, int32_t accumulate) {
+    MB_CTX(ctx);
+    if (!A || !B) return fail(MB_ERR_INVALID_ARG, "multDenseSparse: null operand");
+    if (A->cols != B->rows) return fail(MB_ERR_DIM_MISMATCH, "matrix dimension mismatch: %d v.s %d", A->cols, B->rows);
+    int32_t r = dense_f64(A, "multDenseSparse");
+    if (r) return r;
+    if ((r = check_out(C, A->rows, B->cols, "multDenseSparse"))) return r;
+    int launches = 0;
+    MB_CUDA(mb::spmm_dense_sparse(f64_ptr(A), rs(A), cs(A), A->rows, B->col_ptr, B->row_idx, B->val, B->cols, f64_ptr(C), rs(C),
+                                  cs(C), accumulate ? 1 : 0, ctx->stream, &launches));
+    ctx->launches += launches;
+    return MB_OK;
+}
+
+int32_t mb_spmm_sparse_dense(mb_ctx* ctx, const mb_spblock* A, const mb_block* B, mb_block* C, int32_t accumulate) {
+    MB_CTX(ctx);
+    if (!A || !B) return fail(MB_ERR_INVALID_ARG, "multSparseDense: null operand");
+    if (A->cols != B->rows) return fail(MB_ERR_DIM_MISMATCH, "matrix dimension mismatch: %d v.s %d", A->cols, B->rows);
+    int32_t r = dense_f64(B, "multSparseDense");
+    if (r) return r;
+    if ((r = check_out(C, A->rows, B->cols, "multSparseDense"))) return r;
+    tile_ws ws;
+    ws.st = ctx->stream;
+    const long long need = mb::sparse_tile_ptr_ints(A->rows, A->cols);
+    if (need > 0 && B->cols > 0) MB_CUDA(cudaMallocAsync(&ws.p, sizeof(int) * (size_t)need, ctx->stream));
+    int launches = 0;
+    MB_CUDA(mb::spmm_sparse_dense(A->col_ptr, A->row_idx, A->val, A->rows, A->cols, f64_ptr(B), rs(B), cs(B), B->cols, f64_ptr(C),
+                                  rs(C), cs(C), accumulate ? 1 : 0, ws.p, ctx->stream, &launches));
+    ctx->launches += launches;
+    return MB_OK;
+}
+
+int32_t mb_spgemm_to_dense(mb_ctx* ctx, const mb_spblock* A, const mb_spblock* B, mb_block* C, int32_t accumulate) {
+    MB_CTX(ctx);
+    if (!A || !B) return fail(MB_ERR_INVALID_ARG, "SparseMatrix.multiply: null operand");
+    if (A->cols != B->rows) return fail(MB_ERR_DIM_MISMATCH, "matrix dimension mismatch: %d v.s %d", A->cols, B->rows);
+    int32_t r = check_out(C, A->rows, B->cols, "SparseMatrix.multiply");
+    if (r) return r;
+    tile_ws ws;
+    ws.st = ctx->stream;
+    const long long need = mb::sparse_tile_ptr_ints(A->rows, A->cols);
+    if (need > 0 && B->cols > 0) MB_CUDA(cudaMallocAsync(&ws.p, sizeof(int) * (size_t)need, ctx->stream));
+    int launches = 0;
+    MB_CUDA(mb::spgemm_to_dense(A->col_ptr, A->row_idx, A->val, A->rows, A->cols, B->col_ptr, B->row_idx, B->val, B->cols,
+                                f64_ptr(C), rs(C), cs(C), accumulate ? 1 : 0, ws.p, ctx->stream, &launches));
+    ctx->launches += launches;
+    return MB_OK;
+}
+
 }  // extern "C"
+

@@ -5,6 +5,8 @@
 #include <cstdint>
 #include <cstring>
 
+int32_t mb_fail(int32_t code, const char* fmt, ...);   // capi.cu: sets mb_last_error()
+
 namespace {
 
 // utils/MTUtils.scala:204-213
@@ -145,6 +147,43 @@ int32_t mb_partition_seeds(int64_t seed, int32_t num_partitions, int64_t* seeds_
         const int64_t lo = int64_t(next32());
         seeds_out[i] = int64_t((uint64_t(hi) << 32) + uint64_t(lo));   // ((long)next(32) << 32) + next(32)
     }
+    return MB_OK;
+}
+
+// matrix/Matrices.scala:57-104 (SparseMatrix as one SparseVector per column) as CSC.  Checked before any upload.
+int32_t mb_csc_check(int32_t rows, int32_t cols, const int32_t* col_ptr, const int32_t* row_idx) {
+    if (rows < 0 || cols < 0) return mb_fail(MB_ERR_INVALID_ARG, "sparse block: negative dimension %d x %d", rows, cols);
+    if (!col_ptr) return mb_fail(MB_ERR_INVALID_ARG, "sparse block: null col_ptr");
+    if (col_ptr[0] != 0) return mb_fail(MB_ERR_INVALID_ARG, "sparse block: col_ptr[0] = %d, expected 0", col_ptr[0]);
+    for (int32_t c = 0; c < cols; ++c)
+        if (col_ptr[c + 1] < col_ptr[c])
+            return mb_fail(MB_ERR_INVALID_ARG, "sparse block: col_ptr decreases at column %d (%d > %d)", c, col_ptr[c],
+                           col_ptr[c + 1]);
+    if (col_ptr[cols] > 0 && !row_idx) return mb_fail(MB_ERR_INVALID_ARG, "sparse block: null row_idx");
+    for (int32_t c = 0; c < cols; ++c) {
+        for (int32_t p = col_ptr[c]; p < col_ptr[c + 1]; ++p) {
+            if (row_idx[p] < 0 || row_idx[p] >= rows)
+                return mb_fail(MB_ERR_INVALID_ARG, "sparse block: row index %d of column %d outside [0, %d)", row_idx[p], c, rows);
+            if (p > col_ptr[c] && row_idx[p] <= row_idx[p - 1])
+                return mb_fail(MB_ERR_INVALID_ARG, "sparse block: row indices of column %d not strictly increasing (%d after %d)",
+                               c, row_idx[p], row_idx[p - 1]);
+        }
+    }
+    return MB_OK;
+}
+
+// matrix/Matrices.scala:157-173: sparseSize = (numCols * sparsity).toInt
+int32_t mb_sparse_rand_count(int32_t rows, int32_t cols, double sparsity, int32_t* count) {
+    if (!count || rows < 0 || cols < 0) return mb_fail(MB_ERR_INVALID_ARG, "SparseMatrix.rand: bad argument");
+    if (!(sparsity >= 0.0)) return mb_fail(MB_ERR_INVALID_ARG, "SparseMatrix.rand: sparsity %g must be >= 0", sparsity);
+    const double want = double(cols) * sparsity;
+    if (want >= 2147483648.0) return mb_fail(MB_ERR_INVALID_ARG, "SparseMatrix.rand: %g entries per column", want);
+    const int32_t s = int32_t(want);
+    if (s > rows)
+        return mb_fail(MB_ERR_INVALID_ARG, "SparseMatrix.rand: %d distinct rows per column requested from %d rows", s, rows);
+    if (int64_t(s) * cols >= (int64_t(1) << 31))
+        return mb_fail(MB_ERR_INVALID_ARG, "SparseMatrix.rand: %lld entries, larger than Int.MaxValue", (long long)s * cols);
+    *count = s;
     return MB_OK;
 }
 

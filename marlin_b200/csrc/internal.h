@@ -54,6 +54,16 @@ struct mb_block {
     void* ready_event = nullptr;   // optional cudaEvent_t: the block's contents are final once it has completed
 };
 
+// CSC sparse block (include/marlin_b200.h): device arrays owned by the record; row_idx / val are null when nnz == 0
+struct mb_spblock {
+    int rows = 0, cols = 0;
+    long long nnz = 0;
+    int* col_ptr = nullptr;
+    int* row_idx = nullptr;
+    double* val = nullptr;
+    int device = 0;
+};
+
 namespace mb {
 cudaError_t ipc_export(const void* dptr, unsigned char handle[64], long long* offset, long long* alloc_bytes);
 cudaError_t ipc_open(const unsigned char handle[64], void** base_out);

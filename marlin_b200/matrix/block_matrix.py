@@ -77,6 +77,25 @@ class BlockMatrix(DistributedMatrix):
     def getBlocks(self):
         return self.blocks
 
+    # ------------------------------------------------------------------ sparse blocks
+    def _any_sparse(self) -> bool:
+        """Whether any block of this matrix (on any rank) is sparse; agreed once per matrix (blocks are immutable)."""
+        if getattr(self, "_sparse", None) is None:
+            self._sparse = any(self._all_gather_meta([any(s.isSparse for _, s in self.blocks)]))
+        return self._sparse
+
+    def _require_dense(self, op: str, *others) -> None:
+        """The reference dereferences `denseBlock` here, which is null for a sparse block."""
+        for m in (self,) + others:
+            if isinstance(m, BlockMatrix) and m._any_sparse():
+                raise nat.MarlinArgumentError(nat.MB_ERR_UNSUPPORTED, f"{op} is not supported on a BlockMatrix with sparse "
+                                              "blocks: convert it with toDenseBlocks first")
+
+    def toDenseBlocks(self) -> "BlockMatrix":
+        """:596-603 — every sparse block becomes `new SubMatrix(denseMatrix = sparseBlock.toDense)` on its GPU."""
+        res = [(b, s.toDenseBlock()) for b, s in self.blocks]
+        return BlockMatrix(res, self._nRows, self._nCols, self._blksByRow, self._blksByCol, self._placement)
+
     def owner(self, row: int, col: int) -> int:
         """Rank holding block (row, col): explicit placement or MatrixElemOpPartitioner order mod G."""
         rank, ws = world()
@@ -169,6 +188,7 @@ class BlockMatrix(DistributedMatrix):
                                           f"{self.numCols()} vs {other.numRows()}")
         if self.numBlksByCol() == other.numBlksByRow():
             return self._multiply_same_grid(other)
+        self._require_dense("multiply with a re-split grid (slices of denseBlock, :187-216)", other)
         if self.numBlksByCol() % other.numBlksByRow() == 0:                    # :187-201
             self._check_even_cols()
             ratio = self.numBlksByCol() // other.numBlksByRow()
@@ -201,6 +221,10 @@ class BlockMatrix(DistributedMatrix):
         """:152-186 — m*k*n block products keyed by seq, k-way sum per C tile."""
         m, k, n = self.numBlksByRow(), self.numBlksByCol(), other.numBlksByCol()
         rank, ws = world()
+        sparse = self._any_sparse() or other._any_sparse()
+        if sparse and ws > 1:
+            raise nat.MarlinArgumentError(nat.MB_ERR_UNSUPPORTED, "multiply of a BlockMatrix with sparse blocks runs on one "
+                                          "rank; convert with toDenseBlocks for the multi-GPU multiply")
         plan = comm.plan_multiply(m, k, n, ws, self.owner, other.owner)
         a_local = {(b.row, b.column): s for b, s in self.blocks}
         b_local = {(b.row, b.column): s for b, s in other.blocks}
@@ -245,7 +269,8 @@ class BlockMatrix(DistributedMatrix):
         by_c: Dict[Tuple[int, int], List[int]] = {}
         for (i, j, kk) in mine:
             by_c.setdefault((i, j), []).append(kk)
-        whole = bool(by_c) and all(sorted(v) == list(range(k)) for v in by_c.values())
+        # sparse operands: one sparse-product launch per block product, the kk partials accumulated in place
+        whole = not sparse and bool(by_c) and all(sorted(v) == list(range(k)) for v in by_c.values())
         if whole and len(by_c) <= 16 and k <= 16:
             # this rank holds every kk of its C tiles: ONE grouped persistent launch (K loop concatenated over kk)
             import ctypes as C
@@ -390,6 +415,7 @@ class BlockMatrix(DistributedMatrix):
         row: a running accumulate for the blocks one rank holds, then partials to the rank of block (row, 0).
         The result is labelled with v's length and split count, as the reference does (:252,257)."""
         from .distributed_vector import DistributedVector
+        self._require_dense("matrix x vector multiply")            # SubMatrix.multiply(v: Vector), SubMatrix.scala:131-139
         if self.numCols() != v.length:
             raise nat.MarlinArgumentError(nat.MB_ERR_DIM_MISMATCH, "Dimension mismatch during matrix-matrix multiplication "
                                           f"{self.numCols()} v.s {v.length}")
@@ -412,6 +438,7 @@ class BlockMatrix(DistributedMatrix):
         """multiply(v: BDV[Double]) :265-274 — broadcast vector, the matrix must not be split by column."""
         from .distributed_vector import DistributedVector
         v = np.asarray(v, dtype=np.float64).reshape(-1)
+        self._require_dense("matrix x vector multiply")            # SubMatrix.multiply(v: Vector), SubMatrix.scala:131-139
         if self.numCols() != v.shape[0]:
             raise nat.MarlinArgumentError(nat.MB_ERR_DIM_MISMATCH,
                                           f"matrix columns size {self.numCols()} not support vector length {v.shape[0]}")
@@ -432,6 +459,7 @@ class BlockMatrix(DistributedMatrix):
         numCols() (what the several-block-rows branch at :333 also reports), so the result can be used by the next
         operation.  (2) The column range of B at :324-330 is bounded by numCols(), not by B.cols; when that range runs past
         B.cols Breeze's slice throws, and so does this port (no clamping)."""
+        self._require_dense("multiplyBy")
         Bd = B if isinstance(B, SubMatrix) else SubMatrix(B)
         if Bd.cols != self.numRows():
             raise nat.MarlinArgumentError(nat.MB_ERR_DIM_MISMATCH, "Dimension mismatch during matrix-matrix multiplication: "
@@ -479,6 +507,8 @@ class BlockMatrix(DistributedMatrix):
 
     # ------------------------------------------------------------------ element-wise
     def _scalar(self, op: str, b: float) -> "BlockMatrix":
+        if op in ("subtractBy", "divideBy"):
+            self._require_dense(op)                                          # :416,444 read denseBlock.data
         f = {"add": lambda s: s.add(b), "subtract": lambda s: s.subtract(b), "multiply": lambda s: s.multiply(b),
              "divide": lambda s: s.divide(b), "subtractBy": lambda s: s.subtractBy(b), "divideBy": lambda s: s.divideBy(b)}[op]
         return BlockMatrix([(k, f(v)) for k, v in self.blocks], self.numRows(), self.numCols(), self.numBlksByRow(),
@@ -490,6 +520,7 @@ class BlockMatrix(DistributedMatrix):
             return self._scalar(op, float(other))
         if self.numRows() != other.numRows() or self.numCols() != other.numCols():
             raise nat.MarlinArgumentError(nat.MB_ERR_DIM_MISMATCH, "matrix dimension mismatch")
+        self._require_dense(op, other)
         if isinstance(other, DenseVecMatrix):                                  # :346-349
             return getattr(self.toDenseVecMatrix(), op)(other)
         if self.numBlksByRow() != other.numBlksByRow() or self.numBlksByCol() != other.numBlksByCol():
@@ -546,6 +577,7 @@ class BlockMatrix(DistributedMatrix):
 
     def sum(self) -> float:
         """:467-472"""
+        self._require_dense("sum")
         parts = self._all_gather_meta([s.sum() for _, s in self.blocks])
         if not parts:
             raise nat.MarlinError(nat.MB_ERR_EMPTY, "empty collection")
@@ -556,6 +588,7 @@ class BlockMatrix(DistributedMatrix):
 
     def transpose(self) -> "BlockMatrix":
         """:514-523 — per-block materialised transpose, key (r, c) -> (c, r); no data leaves its GPU."""
+        self._require_dense("transpose")
         res = [(BlockID(b.column, b.row), s.transpose()) for b, s in self.blocks]
         return BlockMatrix(res, self.numCols(), self.numRows(), self.numBlksByCol(), self.numBlksByRow(),
                            placement=lambda r, c, s=self: s.owner(c, r))
@@ -564,12 +597,14 @@ class BlockMatrix(DistributedMatrix):
     def toDenseVecMatrix(self):
         """:575-594 — blocks -> rows.  Rows of block-row r are assembled on owner(r, 0)."""
         from .dense_vec_matrix import DenseVecMatrix
+        self._require_dense("toDenseVecMatrix")
         return DenseVecMatrix._from_block_matrix(self)
 
     def toBlockMatrix(self, newNumByRow: int, newNumByCol: int) -> "BlockMatrix":
         """:610-665 — re-grid.  Pieces are cut as views, shipped once, and pasted into the new blocks."""
         if self._blksByRow == newNumByRow and self._blksByCol == newNumByCol:
             return self
+        self._require_dense("toBlockMatrix (re-grid)")
         nr, nc = self.numRows(), self.numCols()
         rl, cl = _ceil_len(nr, self.numBlksByRow()), _ceil_len(nc, self.numBlksByCol())
         nrl, ncl = _ceil_len(nr, newNumByRow), _ceil_len(nc, newNumByCol)
@@ -627,6 +662,7 @@ class BlockMatrix(DistributedMatrix):
     # ------------------------------------------------------------------ I/O (next-row (f)-3)
     def saveToFileSystem(self, path: str, format: str = " ") -> None:
         """:550-559 — "blockmatrix": `row-col-rows-cols:v,v,...` column-major; else DenseVecMatrix format."""
+        self._require_dense("saveToFileSystem")
         from ..utils.mt_utils import _jdouble
         if format.lower() == "blockmatrix":
             lines = []

@@ -3,7 +3,8 @@
 The reference's SubMatrix wraps a Breeze DenseMatrix[Double] on the JVM heap; here the same
 (data, offset, rows, cols, majorStride, isTranspose) record points into HBM.  The buffer is a torch
 tensor only so that torch.distributed (NCCL) can move it; every arithmetic method calls the C ABI
-of libmarlin_b200.so (the kernel seam named in SURVEY.md §2 #3).  Sparse blocks are out of scope.
+of libmarlin_b200.so (the kernel seam named in SURVEY.md §2 #3).  A sparse block (`SubMatrix(spMatrix=...)`) holds a
+device-resident CSC SparseMatrix instead and dispatches exactly as SubMatrix.scala:41-139 does.
 """
 from __future__ import annotations
 
@@ -22,13 +23,23 @@ _MB_DTYPE = {v: k for k, v in _TORCH_DTYPE.items()}
 Number = Union[int, float]
 
 
+def _unsupported(msg: str) -> nat.MarlinArgumentError:
+    return nat.MarlinArgumentError(nat.MB_ERR_UNSUPPORTED, msg)
+
+
 class SubMatrix:
     """A dense block.  Element (r, c) = buf.flatten()[offset + r + c*ld] (or [offset + c + r*ld] if
-    is_transpose), exactly Breeze's DenseMatrix indexing."""
+    is_transpose), exactly Breeze's DenseMatrix indexing.  Or, built with `spMatrix=`, a sparse block (CSC on the GPU)."""
 
-    def __init__(self, denseMatrix=None, *, buf: Optional[torch.Tensor] = None, rows: int = 0, cols: int = 0,
+    def __init__(self, denseMatrix=None, *, spMatrix=None, buf: Optional[torch.Tensor] = None, rows: int = 0, cols: int = 0,
                  ld: Optional[int] = None, offset: int = 0, is_transpose: bool = False, device=None):
         self._handle = None
+        self._sp = spMatrix
+        if spMatrix is not None:                                            # SubMatrix.scala:22-25
+            self.buf = None
+            self._rows, self._cols = spMatrix.numRows, spMatrix.numCols
+            self.ld, self.offset, self.is_transpose = max(1, self._rows), 0, False
+            return
         if denseMatrix is not None:
             if isinstance(denseMatrix, SubMatrix):
                 src = denseMatrix
@@ -79,24 +90,32 @@ class SubMatrix:
 
     @property
     def isSparse(self) -> bool:
-        return False
+        return self._sp is not None
 
     @property
-    def denseBlock(self) -> "SubMatrix":
-        return self
+    def denseBlock(self) -> Optional["SubMatrix"]:
+        return None if self._sp is not None else self
+
+    @property
+    def sparseBlock(self):
+        return self._sp
 
     @property
     def dtype(self) -> int:
-        return _MB_DTYPE[self.buf.dtype]
+        return nat.MB_F64 if self._sp is not None else _MB_DTYPE[self.buf.dtype]
 
     @property
     def t(self) -> "SubMatrix":
         """Breeze `.t`: a transposed view, no copy."""
+        if self._sp is not None:
+            self.handle()                                                    # raises MB_ERR_UNSUPPORTED
         return SubMatrix(buf=self.buf, rows=self._cols, cols=self._rows, ld=self.ld, offset=self.offset,
                          is_transpose=not self.is_transpose)
 
     def slice(self, r0: int, r1: int, c0: int, c1: int) -> "SubMatrix":
         """Breeze `m(r0 until r1, c0 until c1)`: a view with the parent's majorStride (BlockMatrix.scala:198,299)."""
+        if self._sp is not None:
+            self.handle()                                                    # raises MB_ERR_UNSUPPORTED
         if not (0 <= r0 <= r1 <= self._rows and 0 <= c0 <= c1 <= self._cols):
             raise ValueError("slice out of range")
         rs, cs = (self.ld, 1) if self.is_transpose else (1, self.ld)
@@ -107,7 +126,16 @@ class SubMatrix:
         return (not self.is_transpose) and self.offset == 0 and self.ld == max(1, self._rows)
 
     # ---- native handle ----
+    def _dense_runtime(self) -> Runtime:
+        """The runtime, synchronised to the current stream, for an operation on a dense block."""
+        if self._sp is not None:
+            self.handle()                                                    # raises MB_ERR_UNSUPPORTED
+        rt = Runtime.get(); rt.sync_stream()
+        return rt
+
     def handle(self):
+        if self._sp is not None:
+            raise _unsupported("this operation needs a dense block and this block is sparse: convert with toDenseBlocks")
         if self._handle is None:
             if not self.buf.is_cuda:
                 raise nat.MarlinError(nat.MB_ERR_CUDA, "block lives in host memory: marlin_b200 computes on B200 only "
@@ -126,7 +154,7 @@ class SubMatrix:
         """Record that everything queued so far on the current stream produces this block's FINAL contents (blocks are
         immutable values, like the blocks of a cached RDD): the multi-GPU multiply then offers the block to other ranks as
         soon as this event completes instead of after all later work on the stream (see mb_block_set_ready_event)."""
-        if self.buf.is_cuda:
+        if self._sp is None and self.buf.is_cuda:
             ev = torch.cuda.Event()
             ev.record(torch.cuda.current_stream(self.buf.device))
             self._ready_event = ev
@@ -157,8 +185,17 @@ class SubMatrix:
         return SubMatrix.empty(rows, cols, dtype, self.buf.device)
 
     # ---- arithmetic (matrix/SubMatrix.scala:41-139) ----
+    def _check_dense_pair(self, other: "SubMatrix", op: str) -> None:
+        if self.isSparse or other.isSparse:                                  # :46-48, :66-68
+            raise _unsupported(f"Not supported {op}-operator between matrices of sparsity with {str(self.isSparse).lower()} "
+                               f"and {str(other.isSparse).lower()}")
+
     def add(self, other: Union["SubMatrix", Number]) -> "SubMatrix":
-        rt = Runtime.get(); rt.sync_stream()
+        if isinstance(other, SubMatrix):
+            self._check_dense_pair(other, "add")
+        elif self.isSparse:
+            return SubMatrix(spMatrix=self._sp._map_values(1.0, float(other)))                   # :53-56
+        rt = self._dense_runtime()
         out = self._new_like()
         if isinstance(other, SubMatrix):
             nat.check(rt.lib.mb_block_add(rt.ctx, self.handle(), other.handle(), out.handle()))      # :41-45
@@ -167,7 +204,11 @@ class SubMatrix:
         return out
 
     def subtract(self, other: Union["SubMatrix", Number]) -> "SubMatrix":
-        rt = Runtime.get(); rt.sync_stream()
+        if isinstance(other, SubMatrix):
+            self._check_dense_pair(other, "subtract")
+        elif self.isSparse:
+            return SubMatrix(spMatrix=self._sp._map_values(1.0, -float(other)))                  # :72-75
+        rt = self._dense_runtime()
         out = self._new_like()
         if isinstance(other, SubMatrix):
             nat.check(rt.lib.mb_block_sub(rt.ctx, self.handle(), other.handle(), out.handle()))      # :60-64
@@ -176,35 +217,42 @@ class SubMatrix:
         return out
 
     def divide(self, b: Number) -> "SubMatrix":
-        rt = Runtime.get(); rt.sync_stream()
+        if self.isSparse:
+            return SubMatrix(spMatrix=self._sp._map_values(1.0, 0.0, divide_by=float(b)))       # :80-83
+        rt = self._dense_runtime()
         out = self._new_like()
         nat.check(rt.lib.mb_block_div(rt.ctx, self.handle(), float(b), 0, out.handle()))               # :79-85
         return out
 
     def subtractBy(self, b: Number) -> "SubMatrix":
         """b - x (matrix/BlockMatrix.scala:414-424; returns a new block instead of mutating in place)."""
-        rt = Runtime.get(); rt.sync_stream()
+        rt = self._dense_runtime()
         out = self._new_like()
         nat.check(rt.lib.mb_block_axpb(rt.ctx, self.handle(), -1.0, float(b), out.handle()))
         return out
 
     def divideBy(self, b: Number) -> "SubMatrix":
         """b / x (matrix/BlockMatrix.scala:442-452)."""
-        rt = Runtime.get(); rt.sync_stream()
+        rt = self._dense_runtime()
         out = self._new_like()
         nat.check(rt.lib.mb_block_div(rt.ctx, self.handle(), float(b), 1, out.handle()))
         return out
 
     def elementMultiply(self, other: "SubMatrix") -> "SubMatrix":
-        rt = Runtime.get(); rt.sync_stream()
+        rt = self._dense_runtime()
         out = self._new_like()
         nat.check(rt.lib.mb_block_hadamard(rt.ctx, self.handle(), other.handle(), out.handle()))
         return out
 
     def multiply(self, other, out: Optional["SubMatrix"] = None, accumulate: bool = False,
                  out_dtype: Optional[int] = None) -> "SubMatrix":
-        """:87-111 (block x block, block x local matrix) and :123-131 (scalar)."""
-        rt = Runtime.get(); rt.sync_stream()
+        """:87-111 (block x block, block x local matrix) and :123-131 (scalar).  With a sparse operand the four arms of
+        :88-100 (dense x dense, sparse x sparse, dense x sparse, sparse x dense) and :112-114 (sparse x local matrix)."""
+        if isinstance(other, (int, float)) and self.isSparse:
+            return SubMatrix(spMatrix=self._sp._map_values(float(other), 0.0))                  # :122-125
+        if not isinstance(other, (int, float)) and (self.isSparse or (isinstance(other, SubMatrix) and other.isSparse)):
+            return self._multiply_sparse(other, out, accumulate)
+        rt = self._dense_runtime()
         if isinstance(other, (int, float)):
             res = self._new_like()
             nat.check(rt.lib.mb_block_axpb(rt.ctx, self.handle(), float(other), 0.0, res.handle()))
@@ -219,16 +267,30 @@ class SubMatrix:
         nat.check(rt.lib.mb_block_gemm(rt.ctx, self.handle(), other.handle(), out.handle(), int(accumulate)))
         return out
 
+    def _multiply_sparse(self, other, out: Optional["SubMatrix"], accumulate: bool) -> "SubMatrix":
+        from .sparse_matrix import LibMatrixMult
+        if not isinstance(other, SubMatrix):
+            other = SubMatrix(other)
+        if self.isSparse and other.isSparse:
+            return self._sp.multiply(other._sp, out=out, accumulate=accumulate)            # :92-94
+        if other.isSparse:
+            return LibMatrixMult.multDenseSparse(self, other._sp, out=out, accumulate=accumulate)   # :95-97
+        return LibMatrixMult.multSparseDense(self._sp, other, out=out, accumulate=accumulate)      # :98-100, :112-114
+
+    def toDenseBlock(self) -> "SubMatrix":
+        """`new SubMatrix(denseMatrix = sparseBlock.toDense)` (BlockMatrix.scala:598); a dense block is returned as is."""
+        return self._sp.toDense() if self._sp is not None else self
+
     def dot(self, other: "SubMatrix") -> float:
         """Breeze `v.t * w` of two single-column (or single-row) blocks (matrix/DistributedVector.scala:167)."""
-        rt = Runtime.get(); rt.sync_stream()
+        rt = self._dense_runtime()
         out = C.c_double()
         nat.check(rt.lib.mb_block_dot(rt.ctx, self.handle(), other.handle(), C.byref(out)))
         return float(out.value)
 
     def outer(self, other: "SubMatrix") -> "SubMatrix":
         """Breeze `v * w.t` (matrix/DistributedVector.scala:157): rank-1 block of two vectors."""
-        rt = Runtime.get(); rt.sync_stream()
+        rt = self._dense_runtime()
         n0 = self._rows * self._cols
         n1 = other._rows * other._cols
         out = SubMatrix.empty(n0, n1, nat.MB_F64, self.buf.device)
@@ -239,7 +301,7 @@ class SubMatrix:
     def lu(self):
         """`brzLU(m)` (matrix/DenseVecMatrix.scala:302): (packed unit-lower L and U, permutation array with the
         reference's meaning: row i of L*U is row perm[i] of this block)."""
-        rt = Runtime.get(); rt.sync_stream()
+        rt = self._dense_runtime()
         out = self.copy()
         perm = (C.c_int32 * max(1, self._rows))()
         nat.check(rt.lib.mb_block_lu(rt.ctx, out.handle(), perm))
@@ -247,52 +309,52 @@ class SubMatrix:
 
     def cholesky(self) -> "SubMatrix":
         """`brzCholesky(m)` (:495,513): lower L with L L^T = this, zeros above the diagonal."""
-        rt = Runtime.get(); rt.sync_stream()
+        rt = self._dense_runtime()
         out = self.copy()
         nat.check(rt.lib.mb_block_cholesky(rt.ctx, out.handle()))
         return out
 
     def inverse(self) -> "SubMatrix":
         """`brzInv(m)` (:587,606)."""
-        rt = Runtime.get(); rt.sync_stream()
+        rt = self._dense_runtime()
         out = SubMatrix.empty(self._rows, self._cols, nat.MB_F64, self.buf.device)
         nat.check(rt.lib.mb_block_inverse(rt.ctx, self.handle(), out.handle()))
         return out
 
     def solveTriangular(self, rhs: "SubMatrix", lower: bool, unit: bool = False) -> "SubMatrix":
         """`this \\ rhs` for a triangular `this` (the `l \\ ...` of :364): returns X with this * X = rhs."""
-        rt = Runtime.get(); rt.sync_stream()
+        rt = self._dense_runtime()
         x = rhs.copy()
         nat.check(rt.lib.mb_block_trsm(rt.ctx, self.handle(), int(lower), int(unit), x.handle()))
         return x
 
     def add_(self, other: "SubMatrix") -> "SubMatrix":
         """In-place accumulate (the reduceByKey combine of BlockMatrix.scala:177 without a new allocation)."""
-        rt = Runtime.get(); rt.sync_stream()
+        rt = self._dense_runtime()
         nat.check(rt.lib.mb_block_add(rt.ctx, self.handle(), other.handle(), self.handle()))
         return self
 
     def transpose(self) -> "SubMatrix":
         """`denseBlock.t.copy` (matrix/BlockMatrix.scala:517): materialised transpose."""
-        rt = Runtime.get(); rt.sync_stream()
+        rt = self._dense_runtime()
         out = SubMatrix.empty(self._cols, self._rows, self.dtype, self.buf.device)
         nat.check(rt.lib.mb_block_transpose(rt.ctx, self.handle(), out.handle()))
         return out
 
     def copy(self, dtype: Optional[int] = None) -> "SubMatrix":
         """Breeze `.copy`: packed column-major copy of a view (optionally converting fp64 <-> bf16/fp32)."""
-        rt = Runtime.get(); rt.sync_stream()
+        rt = self._dense_runtime()
         out = SubMatrix.empty(self._rows, self._cols, self.dtype if dtype is None else dtype, self.buf.device)
         nat.check(rt.lib.mb_block_copy(rt.ctx, self.handle(), out.handle()))
         return out
 
     def assign(self, src: "SubMatrix") -> None:
         """`this(range) := src` — copy src into this view."""
-        rt = Runtime.get(); rt.sync_stream()
+        rt = self._dense_runtime()
         nat.check(rt.lib.mb_block_copy(rt.ctx, src.handle(), self.handle()))
 
     def sum(self) -> float:
-        rt = Runtime.get(); rt.sync_stream()
+        rt = self._dense_runtime()
         blk = self if self.dtype == nat.MB_F64 else self.copy(nat.MB_F64)
         out = C.c_double()
         nat.check(rt.lib.mb_block_sum(rt.ctx, blk.handle(), C.byref(out)))
@@ -300,7 +362,9 @@ class SubMatrix:
 
     # ---- host transfer (toBreeze / collect) ----
     def toBreeze(self) -> np.ndarray:
-        """Download as a (rows x cols) Fortran-ordered float64 ndarray."""
+        """Download as a (rows x cols) Fortran-ordered float64 ndarray (a sparse block is densified)."""
+        if self._sp is not None:
+            return self._sp.toDense().toBreeze()
         if self._rows == 0 or self._cols == 0:
             return np.zeros((self._rows, self._cols), order="F")
         if self.buf.is_cuda:
@@ -317,6 +381,8 @@ class SubMatrix:
     to_numpy = toBreeze
 
     def __repr__(self):
+        if self._sp is not None:
+            return f"SubMatrix(sparse {self._sp!r})"
         return f"SubMatrix({self._rows}x{self._cols}, ld={self.ld}, t={self.is_transpose}, {self.buf.dtype}, {self.buf.device})"
 
 

@@ -21,6 +21,7 @@ from .. import comm
 from ..matrix.block import BlockID
 from ..matrix.block_matrix import BlockMatrix
 from ..matrix.dense_vec_matrix import DenseVecMatrix
+from ..matrix.sparse_matrix import SparseMatrix
 from ..matrix.sub_matrix import SubMatrix
 from ..runtime import Runtime, world
 
@@ -125,9 +126,13 @@ class MTUtils:
                           distribution: Optional[UniformGenerator] = None, seed: Optional[int] = None,
                           dtype: int = nat.MB_F64) -> BlockMatrix:
         """utils/MTUtils.scala:34-50 -> RandomBlockRDD (rdd/RandomRDD.scala:184-223): one partition per block in
-        row-major BlockID order, `BDM.create(rows, cols, Array.fill(rows*cols)(nextValue()))` (column-major)."""
-        if sparseInfo[0]:
-            raise nat.MarlinArgumentError(nat.MB_ERR_UNSUPPORTED, "sparse blocks are out of scope")
+        row-major BlockID order, `BDM.create(rows, cols, Array.fill(rows*cols)(nextValue()))` (column-major).
+        sparseInfo = (True, d): every block is `SparseMatrix.rand(rows, cols, d)` (rdd/RandomRDD.scala:97-100),
+        generated on the GPU from the block's partition seed, so a seed reproduces the matrix (the reference's sparse
+        generator is unseeded); values are U[0,1) and `distribution` does not apply, as in the reference."""
+        sparse, density = bool(sparseInfo[0]), float(sparseInfo[1])
+        if sparse and dtype != nat.MB_F64:
+            raise nat.MarlinArgumentError(nat.MB_ERR_UNSUPPORTED, "sparse blocks are fp64")
         dist_ = distribution or UniformGenerator(0.0, 1.0)
         brs = int(math.ceil(float(nRows) / float(numByRow)))
         bcs = int(math.ceil(float(nColumns) / float(numByCol)))
@@ -147,6 +152,9 @@ class MTUtils:
             cols = bcs
             if (idx + 1) % by_col == 0 and bcs * by_col > nColumns:
                 cols = nColumns - bcs * (by_col - 1)
+            if sparse:
+                blocks.append((BlockID(i, j), SubMatrix(spMatrix=SparseMatrix.rand(rows, cols, density, seed=seeds[idx]))))
+                continue
             blk = SubMatrix.empty(rows, cols, nat.MB_F64)
             MTUtils._fill(blk, seeds[idx], 0, dist_, row_major=False)
             if dtype != nat.MB_F64:
